@@ -2,6 +2,7 @@
 """Benchmark of the rigid-ICP hot path (BASELINE.json metric: ICP iterations/s and correspondences/s).
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--no-secondary]
+                    [--dump-outputs DIR]
 
 A "step" is one full ICP iteration (transform + radius-bounded 1-NN of every source point + moment accumulation +
 reduction (+ all-reduce) + solve) on the named workload.
@@ -24,6 +25,9 @@ the iteration's kernels, with an L2 flush (256 MiB memset) before every iteratio
 ranks. The timed call starts like every ICP run: its first iteration searches every query (nothing cached), later
 iterations re-search only the queries whose cached match cannot be proven to still be the nearest neighbour
 (icp_loop.cu) - `roofline` reports the mean and both regimes.
+--dump-outputs DIR writes what that timed call returned after its last step (DIR/T.npy, the 3 x 4 float32 transform,
+and the float64 scalars DIR/num_corr.npy, iterations.npy, last_delta.npy, converged.npy); the inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 Parity inside the bench: the GPU transform is compared with the CPU arm's (same inputs, same iteration count), the
 correspondence counts must be equal, all ranks must hold bit-identical transforms, and at N > 1 the sharded result
 is compared with a single-GPU run of the whole problem on rank 0.
@@ -269,13 +273,22 @@ def timed_estimate(icp, ctx, cdist, world, steps, warmup, flush, kw):
     return res, ms_total / steps, wall
 
 
+def dump_outputs(path, res):
+    """The timed estimate()'s result as its caller receives it: the transform and the counts of the last step."""
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "T.npy"), np.asarray(res["T"], np.float32))
+    for key in ("num_corr", "iterations", "last_delta", "converged"):
+        np.save(os.path.join(path, f"{key}.npy"), np.float64(res[key]))
+
+
 def t_hash(T):
     return hashlib.sha1(np.ascontiguousarray(T, np.float32).tobytes()).hexdigest()[:16]
 
 
 def icp_bench(args, name, w, scaling, ctx, rank, world, local, with_e2e=True, with_cpu=True, with_survey=True,
-              clocks_wanted=True):
-    """The ICP legs on `ctx` (all ranks call it); rank 0 gets the JSON-able dict, the others None."""
+              clocks_wanted=True, dump_dir=None):
+    """The ICP legs on `ctx` (all ranks call it); rank 0 gets the JSON-able dict, the others None.
+    dump_dir: where rank 0 writes the timed call's outputs (dump_outputs)."""
     from cilantro_b200 import capi, dist as cdist, synth
 
     flush = not args.no_flush
@@ -296,6 +309,8 @@ def icp_bench(args, name, w, scaling, ctx, rank, world, local, with_e2e=True, wi
     if rank == 0 and clocks_wanted:
         sampler.start()
     res, ms_per_step, wall = timed_estimate(icp, ctx, cdist, world, args.steps, args.warmup, flush, kw)
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, res)
     launches = res["kernel_launches"]  # this library's kernels launched by the timed estimate() call (not the warm-up)
     iter_ms = np.array([cdist.max_over_ranks(x) for x in res["iter_ms"]])
     clocks = None
@@ -500,7 +515,8 @@ def run_ours(args):
     cdist.attach_comm(ctx)
     name, scaling = pick_workload(args)
     w = WORKLOADS[name]
-    main = icp_bench(args, name, w, scaling, ctx, rank, world, local, with_cpu=not args.no_cpu_baseline)
+    main = icp_bench(args, name, w, scaling, ctx, rank, world, local, with_cpu=not args.no_cpu_baseline,
+                     dump_dir=args.dump_outputs)
 
     # ---- secondary workloads ------------------------------------------------------------------------------------
     secondary = {}
@@ -570,7 +586,13 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the `secondary` block (other BASELINE configs)")
     ap.add_argument("--no-flush", action="store_true",
                     help="experiments only: skip the L2 flush between timed iterations (the reported config says so)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the timed ICP call's outputs (transform and counts of its last step) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload in AUX):
+        ap.error("--dump-outputs applies to the ICP workloads of --impl ours")
     args.warmup = max(args.warmup, 0)
     if args.workload in AUX:  # secondary single-GPU workloads (k-means, RANSAC, PCA, ...) on their own: bench_aux.py
         if int(os.environ.get("RANK", "0")) == 0:

@@ -3,7 +3,8 @@ examples/test_clouds/test.ply) — on the committed fixture tests/golden/config1
 at 12 mm by the oracle; tests/golden/make_config1_fixture.py).
 
 CPU part: the oracle runs the example's recipe (rigid_icp.cpp:25-65, settings :119-123) and recovers tf_ref^-1 — the
-self-checking property the example prints; where /root/reference exists the fixture is regenerated and compared.
+self-checking property the example prints; a crop of the scan itself (tests/golden/scan_crop.ply) must downsample to
+exactly the fixture's rows of the voxels it covers.
 GPU part: the same recipe through the C ABI against the oracle: transforms within 1e-5, neighbour indices and residuals
 bit-exact, plus downsampling and normal estimation on real scan data.
 """
@@ -14,6 +15,7 @@ import pytest
 
 from cilantro_b200 import synth
 from conftest import frob
+from golden import make_ref_golden as ref_golden
 
 FIXTURE = os.path.join(os.path.dirname(__file__), "golden", "config1_cloud.npz")
 # icp.setMaxNumberOfOptimizationStepIterations(1).setPointToPointMetricWeight(0).setPointToPlaneMetricWeight(1);
@@ -30,16 +32,17 @@ def test_fixture_matches_the_reference_scan(orc):
     pts, nrm, n_source, n5 = _scan()
     assert pts.shape == nrm.shape and pts.shape[0] > 40000 and n_source == 573663
     assert np.all(np.abs(np.linalg.norm(nrm, axis=1) - 1) < 1e-4)
-    if not os.path.exists("/root/reference/examples/test_clouds/test.ply"):
-        pytest.skip("no /root/reference on this machine: fixture content checked where it was made")
     from golden.make_config1_fixture import read_test_ply
 
-    p, n, c = read_test_ply()
-    assert p.shape[0] == n_source
-    assert orc.grid_downsample(p, 0.005, normals=n, colors=c)[0].shape[0] == n5
+    crop = ref_golden.load()["scan_crop"]  # the scan's vertices inside a box of whole 12 mm voxels, in file order
+    p, n, c = read_test_ply(ref_golden.CROP)
+    assert p.shape[0] == crop["n_vertices"] and 0 < p.shape[0] < n_source
+    assert orc.grid_downsample(p, 0.005, normals=n, colors=c)[0].shape[0] == crop["n_bins_5mm"]
     p12, n12, _ = orc.grid_downsample(p, 0.012, normals=n)
-    assert np.array_equal(p12.view(np.uint32), pts.view(np.uint32))
-    assert np.array_equal(n12.view(np.uint32), nrm.view(np.uint32))
+    rows = crop["fixture_rows"]
+    assert len(rows) > 100 and p12.shape[0] == len(rows)
+    assert np.array_equal(p12.view(np.uint32), pts[rows].view(np.uint32))
+    assert np.array_equal(n12.view(np.uint32), nrm[rows].view(np.uint32))
 
 
 def test_oracle_runs_the_example_recipe(orc):

@@ -1,14 +1,15 @@
 """GPU parity: grid nearest-neighbour search vs the oracle (bit-exact indices and squared distances).
 
 Calls go through the C ABI (cb_knn1_radius / cb_find_correspondences / cb_knn_radius). Oracle:
-orc.BruteKnn (restatement; lowest index wins exact ties — the same rule as the CUDA path) and,
-where oracle/_ref exists, the reference's own nanoflann (ties may pick another index with a
-bit-equal d2).
+orc.BruteKnn (restatement; lowest index wins exact ties — the same rule as the CUDA path) and
+the answers of the reference's own nanoflann stored in tests/golden/ref_nanoflann.json (ties may
+pick another index with a bit-equal d2).
 """
 import numpy as np
 import pytest
 
 from cilantro_b200 import synth
+from golden import make_ref_golden as ref_golden
 
 pytestmark = pytest.mark.gpu
 FMAX = float(np.finfo(np.float32).max)
@@ -107,18 +108,17 @@ def test_find_correspondences_matches_oracle(cb, ctx, orc):
     assert np.all(np.diff(i2) > 0), "correspondences must be compacted in query order"
 
 
-def test_knn1_vs_reference_nanoflann_250k(cb, ctx, orc):
+def test_knn1_vs_reference_nanoflann_250k(cb, ctx):
     """Against the reference's own kd-tree: equal index, or an exact tie (bit-equal d2)."""
-    if not orc.have_ref():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
+    want = ref_golden.load()["knn1_250k"]
     dst, src, _, T_ref = synth.icp_pair(250000, seed=1, noise=0.001)
     T = T_ref.astype(np.float32)
     max_d2 = np.float32(0.02**2)
     idx, d2 = cb.knn1_radius(ctx, cb.Cloud(ctx, dst), cb.Cloud(ctx, src), T, max_d2)
-    ri, rd = orc.RefKnn(dst).query(orc.transform_points(T, src), max_d2)
-    assert np.array_equal(d2.view(np.uint32), rd.view(np.uint32))
-    diff = idx != ri
-    assert diff.sum() <= 5, f"{diff.sum()} index differences (only exact ties may differ)"
+    assert ref_golden.sha(d2) == want["d2"]
+    # the reference's list with its exact ties resolved to the lowest index (the CUDA path's rule), and few such ties
+    assert ref_golden.sha(idx) == want["idx"]
+    assert want["ties"] <= 5, f"{want['ties']} index differences (only exact ties may differ)"
 
 
 def test_knn_k_matches_numpy(cb, ctx):
@@ -184,21 +184,17 @@ def test_radius_search_matches_oracle_bitexact(cb, ctx, orc):
     assert off[-1] == 0
 
 
-def test_radius_search_agrees_with_reference_nanoflann(cb, ctx, orc):
-    if not orc.have_ref():
-        pytest.skip("oracle/_ref not built")
+def test_radius_search_agrees_with_reference_nanoflann(cb, ctx):
+    want = ref_golden.load()["radius_15k"]
     rng = np.random.default_rng(23)
     dst = rng.random((15000, 3), dtype=np.float32)
     qry = rng.random((800, 3), dtype=np.float32)
     r2 = 0.05**2
     off, idx, d2 = cb.radius_search(ctx, cb.Cloud(ctx, dst), cb.Cloud(ctx, qry), r2)
-    ref = orc.RefKnn(dst)
-    _, _, cnt = ref.neighborhoods(qry, 0, r2, stride=1)
-    ri, rd, cnt = ref.neighborhoods(qry, 0, r2, stride=int(cnt.max()))
-    assert np.array_equal(np.diff(off), cnt.astype(np.int64))
-    for i in range(qry.shape[0]):  # random data: no equal distances, so the order is unique
-        assert np.array_equal(idx[off[i]:off[i + 1]], ri[i, :cnt[i]])
-        assert np.array_equal(d2[off[i]:off[i + 1]].view(np.uint32), rd[i, :cnt[i]].view(np.uint32))
+    assert ref_golden.sha(np.diff(off).astype(np.int64)) == want["cnt"]
+    # the rows one after the other; random data: no equal distances, so the order is unique
+    assert ref_golden.sha(idx.astype(np.int64)) == want["idx"]
+    assert ref_golden.sha(d2.astype(np.float32)) == want["d2"]
 
 
 def _hollow_sphere(n, seed=0, radius=0.45, noise=0.002):
@@ -248,6 +244,7 @@ def test_far_queries_cross_empty_space_exactly_and_fast(cb, ctx, orc):
 
 def test_normals_with_isolated_outliers(cb, ctx, orc):
     # scanner outliers far from the surface ask for k neighbours across empty space
+    want = ref_golden.load()["normals_outliers_300k"]
     pts, _ = synth.surface_cloud(300_000, seed=8, noise=0.0005)
     rng = np.random.default_rng(9)
     outliers = (np.array([0.5, 0.5, 0.5]) + 3.0 * rng.standard_normal((25, 3))).astype(np.float32)
@@ -255,22 +252,17 @@ def test_normals_with_isolated_outliers(cb, ctx, orc):
     got = cb.Cloud(ctx, cloud).estimate_normals(k=10, view_point=[0.5, 0.5, 10.0], want_cov=True)
     # Neighbourhoods: the reference's nanoflann for the surface points; brute force (ascending (d2, index), the
     # CUDA path's rule) for the outliers, whose ~10 nearest surface points are several units away and so tie in
-    # fp32 d2 — the one case where the reference's order is its kd-tree traversal order (DESIGN.md §4.7).
-    knn = orc.make_knn(cloud)
-    idx, d2, cnt = knn.neighborhoods(cloud, 10, orc.FLT_MAX)
-    bi, bd, bc = orc.BruteKnn(cloud).neighborhoods(outliers, 10, orc.FLT_MAX)
-    m = pts.shape[0]
-    assert np.array_equal(np.sort(d2[m:], axis=1).view(np.uint32), bd.view(np.uint32))  # same distances either way
-    idx[m:], cnt[m:] = bi, bc
-    want = orc.estimate_normals(cloud, knn, k=10, view_point=[0.5, 0.5, 10.0], neighbors=(idx, cnt))
+    # fp32 d2 — the one case where the reference's order is its kd-tree traversal order (DESIGN.md §4.7). The oracle's
+    # covariances of those neighbourhoods are stored (tests/golden/make_ref_golden.py: outlier_normals_entry).
+    _, bd, _ = orc.BruteKnn(cloud).neighborhoods(outliers, 10, orc.FLT_MAX)
+    assert ref_golden.sha(bd) == want["outlier_d2"]  # the reference's distances, sorted, are the same
     # at 300 k points a couple of surface rows hold two neighbours with bit-equal d2 as well (probability
     # ~ ulp / spacing per pair): bit-exact wherever the distances are distinct, fp32 rounding elsewhere
     # (k + 1 distances: a tie between the 10th and the excluded 11th neighbour changes the SET, not just the order)
-    d11 = knn.neighborhoods(cloud, 11, orc.FLT_MAX)[1]
-    tied = (np.diff(d11, axis=1) == 0).any(axis=1)
-    tied[m:] = False  # the outliers' rows were rebuilt with the shared tie rule
+    tied = np.zeros(cloud.shape[0], bool)
+    tied[want["tied"]] = True
     assert tied.sum() < 20
-    assert np.array_equal(got["cov6"][~tied].view(np.uint32), want[2][~tied].view(np.uint32))
+    assert ref_golden.sha(got["cov6"][~tied]) == want["cov"]
     assert np.isfinite(got["cov6"][tied]).all()  # a legitimate alternative neighbourhood: nothing more to compare
 
 

@@ -53,30 +53,25 @@ def test_fraction_and_one_to_one(orc):
 
 def test_first_to_second_search_pinned_on_reference_nanoflann(orc):
     """FIRST_TO_SECOND / BOTH rebuild a kd-tree over the transformed source on every call
-    (correspondence_search_kd_tree.hpp:195-204, :214-226). With oracle/_ref that search is the reference's own nanoflann
-    (tree built and queried per call); the brute-force restatement the GPU tests compare against must give the same
-    lists on data without exact ties, and the same ICP transforms."""
-    import pytest
-
-    if not orc.have_ref():
-        pytest.skip("oracle/_ref not built (no /root/reference on this machine)")
+    (correspondence_search_kd_tree.hpp:195-204, :214-226). With the reference's own nanoflann doing that search (tree
+    built and queried per call; its lists and ICP transform stored in tests/golden/ref_nanoflann.json), the brute-force
+    restatement the GPU tests compare against must give the same lists on data without exact ties, and the same ICP
+    transforms."""
     from cilantro_b200 import synth
+    from golden import make_ref_golden as ref_golden
 
+    g = ref_golden.load()
     dst, src, _, T_ref = synth.icp_pair(20000, seed=4, noise=0.003, n_src=15000)
     T0 = (0.7 * np.asarray(T_ref) + 0.3 * np.hstack([np.eye(3), np.zeros((3, 1))])).astype(np.float32)
     max_d2 = np.float32((2.0 * 20000 ** (-1.0 / 3.0)) ** 2)
-    knn = orc.RefKnn(dst)
-    for mode in (dict(search_dir="first_to_second"), dict(search_dir="first_to_second", one_to_one=True),
-                 dict(search_dir="both"), dict(search_dir="both", require_reciprocal=True, inlier_fraction=0.7)):
-        a = orc.engine_correspondences(dst, src, T0, knn, max_d2, f2s_reference=True, **mode)
+    for mode, want in zip(ref_golden.ENGINE_MODES, g["engine_f2s"]):
         b = orc.engine_correspondences(dst, src, T0, orc.BruteKnn(dst), max_d2, f2s_reference=False, **mode)
-        assert len(a[0]) > 1000
-        assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1])
-        assert np.array_equal(a[2].view(np.uint32), b[2].view(np.uint32))
-    kw = dict(metric="p2p", max_iter=6, tol=0.0, max_d2=max_d2, search_dir="both", require_reciprocal=True)
-    ra = orc.icp(dst, src, knn, f2s_reference=True, **kw)
-    rb = orc.icp(dst, src, orc.BruteKnn(dst), f2s_reference=False, **kw)
-    assert ra["num_corr"] == rb["num_corr"] and np.array_equal(ra["T"], rb["T"])
+        assert want["n"] > 1000 and len(b[0]) == want["n"]
+        assert ref_golden.sha(b[0]) == want["first"] and ref_golden.sha(b[1]) == want["second"]
+        assert ref_golden.sha(b[2]) == want["value"]
+    rb = orc.icp(dst, src, orc.BruteKnn(dst), f2s_reference=False, max_d2=max_d2, **ref_golden.ENGINE_ICP)
+    assert rb["num_corr"] == g["engine_icp"]["num_corr"]
+    assert np.array_equal(rb["T"], np.float32(g["engine_icp"]["T"]).reshape(3, 4))
 
 
 def test_engine_icp_recovers_a_shift(orc):

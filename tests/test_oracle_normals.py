@@ -1,11 +1,12 @@
 """CPU: the normal-estimation oracle (oracle/cilantro_oracle.cpp: orc_normals_from_neighbors) against known
-answers and, where oracle/_ref exists, with neighbourhoods from the reference's own nanoflann.
+answers and against the neighbourhoods of the reference's own nanoflann (tests/golden/ref_nanoflann.json).
 
 Reference behaviour under test: core/normal_estimation.hpp:279-332 (normals, view-point flip), :357-421
 (curvature), core/covariance.hpp:83-138 (subset mean / covariance, min sample size 3).
 """
 import numpy as np
-import pytest
+
+from golden import make_ref_golden as ref_golden
 
 
 def _plane_cloud(n, normal, seed=0, noise=0.0):
@@ -61,22 +62,18 @@ def test_covariance_matches_numpy_and_min_sample(orc):
 
 
 def test_reference_nanoflann_neighbourhoods_agree_with_brute(orc):
-    if not orc.have_ref():
-        pytest.skip("oracle/_ref not built (no /root/reference on this machine)")
+    g = ref_golden.load()
     rng = np.random.default_rng(5)
     pts = rng.random((5000, 3), dtype=np.float32)
-    brute, ref = orc.BruteKnn(pts), orc.RefKnn(pts)
-    for k, r2 in ((8, orc.FLT_MAX), (16, 0.05**2)):
+    brute = orc.BruteKnn(pts)
+    for (k, r2), want in zip(((8, orc.FLT_MAX), (16, 0.05**2)), g["neighbourhoods_5k"]):
         bi, bd, bc = brute.neighborhoods(pts, k, r2)
-        ri, rd, rc = ref.neighborhoods(pts, k, r2)
-        assert np.array_equal(bc, rc)
-        assert np.array_equal(bd.view(np.uint32), rd.view(np.uint32))
-        assert np.array_equal(bi, ri)  # random data: no exact distance ties
+        assert ref_golden.sha(bc) == want["cnt"]
+        assert ref_golden.sha(bd) == want["d2"]  # bit-equal
+        assert ref_golden.sha(bi) == want["idx"]  # random data: no exact distance ties
     bn = orc.estimate_normals(pts, brute, k=10, view_point=[0.5, 0.5, 3.0])
-    rn = orc.estimate_normals(pts, ref, k=10, view_point=[0.5, 0.5, 3.0])
-    assert np.array_equal(bn[2].view(np.uint32), rn[2].view(np.uint32))  # covariance bit-equal
-    assert np.array_equal(bn[0].view(np.uint32), rn[0].view(np.uint32))
+    assert ref_golden.sha(bn[2]) == g["normals_5k"]["cov"]  # covariance bit-equal
+    assert ref_golden.sha(bn[0]) == g["normals_5k"]["normals"]
     # radius neighbourhoods: same sets (order of exact ties aside)
     _, _, c0 = brute.neighborhoods(pts, 0, 0.04**2, stride=1)
-    _, _, c1 = ref.neighborhoods(pts, 0, 0.04**2, stride=1)
-    assert np.array_equal(c0, c1)
+    assert ref_golden.sha(c0) == g["normals_5k"]["radius_cnt"]
