@@ -98,7 +98,7 @@ EXPORTED = [
     "cb_solve_kabsch_moments", "cb_solve_gauss_newton", "cb_solve_rotation", "cb_compose",
     "cb_kmeans_cluster", "cb_kmeans_assign", "cb_kmeans_seed_indices",
     "cb_ransac_score", "cb_ransac_residuals", "cb_ransac_rigid",
-    "cb_mean_cov", "cb_pca", "cb_transform_points",
+    "cb_mean_cov", "cb_pca", "cb_transform_points", "cb_cloud_segment",
 ]
 
 _lib = None
@@ -595,3 +595,43 @@ def pca(ctx, pts: Cloud):
     evec = np.empty((3, 3), np.float32)
     ok = _check(lib().cb_pca(ctx.h, pts.h, _p(mean), _p(cov), _p(ev), _p(evec)))
     return {"ok": bool(ok), "mean": mean, "cov": cov, "eigenvalues": ev, "eigenvectors": evec}
+
+
+class SegmentParams(C.Structure):
+    _fields_ = [
+        ("k", C.c_int32),
+        ("radius2", C.c_float),
+        ("evaluator", C.c_int32),
+        ("max_distance", C.c_float),
+        ("max_angle", C.c_float),
+        ("color_thresh", C.c_float),
+        ("min_size", C.c_uint64),
+        ("max_size", C.c_uint64),
+    ]
+
+
+SEGMENT_EVALUATORS = {"always_true": 0, "points": 1, "normals": 2, "colors": 3, "points_normals": 4,
+                      "points_colors": 5, "normals_colors": 6, "points_normals_colors": 7}
+
+
+def segment(ctx, cloud: Cloud, k=0, radius2=0.0, evaluator="always_true", max_distance=0.0, max_angle=0.0,
+            color_thresh=0.0, min_size=1, max_size=2**64 - 1, seeds=None, normals=None, colors=None, want_ms=False):
+    """cb_cloud_segment (ConnectedComponentExtraction3f::segment): returns (labels [n] int64, offsets [m + 1] int64,
+    points [offsets[m]] int64, m), plus the stage times [total, neighbourhood + union, finalise] in ms when want_ms.
+    seeds None = every point; normals None = the cloud's own."""
+    n = cloud.n
+    prm = SegmentParams(int(k), float(radius2), SEGMENT_EVALUATORS[evaluator] if isinstance(evaluator, str) else int(evaluator),
+                        float(max_distance), float(max_angle), float(color_thresh), int(min_size), int(max_size))
+    sd = None if seeds is None else np.ascontiguousarray(seeds, np.uint64)
+    nr = None if normals is None else _f32(normals)
+    cl = None if colors is None else _f32(colors)
+    labels = np.empty(max(n, 1), np.uint64)
+    offsets = np.zeros(n + 1, np.uint64)
+    points = np.empty(max(n, 1), np.uint64)
+    m = C.c_size_t()
+    ms = np.zeros(3, np.float32)
+    _check(lib().cb_cloud_segment(ctx.h, cloud.h, C.byref(prm), _p(sd), C.c_size_t(0 if sd is None else sd.shape[0]),
+                                  _p(nr), _p(cl), _p(labels), _p(offsets), _p(points), C.byref(m), _p(ms) if want_ms else None))
+    m = m.value
+    out = (labels[:n].astype(np.int64), offsets[: m + 1].astype(np.int64), points[: int(offsets[m])].astype(np.int64), m)
+    return out + (ms.astype(np.float64),) if want_ms else out

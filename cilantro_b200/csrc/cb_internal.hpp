@@ -160,6 +160,8 @@ int exclusive_scan_u32(cb_context* ctx, uint32_t* d_data, size_t n, uint32_t tot
 int radix_sort_pairs_u64(cb_context* ctx, uint64_t* d_keys, uint32_t* d_vals, uint64_t* d_keys_tmp,
                          uint32_t* d_vals_tmp, size_t n, int bits);
 GridView grid_view(const cb_cloud* c);
+// k-best lists of a cloud against itself, n x k in original order (knn_k.cu; used by segment.cu).
+int knn_lists_self(cb_context* ctx, const cb_cloud* c, int k, float max_d2, int* d_idx, float* d_d2, uint32_t* d_cnt);
 // Scratch for a grid_reduce over `blocks` blocks of `nv` values each (grown on demand).
 int get_reduce_scratch(cb_context* ctx, int blocks, int nv, ReduceScratch* out);
 // Arms the fused exchange for the next pass (bumps ctx->seq) when the tables are ready; returns

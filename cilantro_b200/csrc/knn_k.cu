@@ -75,6 +75,36 @@ __global__ void __launch_bounds__(kBlock) knn_k_kernel(const GridView g, const f
 
 }  // namespace
 
+namespace cb {
+
+// k-best lists of every point of `c` against `c` itself (the neighbourhoods of segment.cu): d_idx / d_d2 are n x k in
+// original order, d_cnt[i] = entries of list i. Stream-ordered; no synchronise.
+int knn_lists_self(cb_context* ctx, const cb_cloud* c, int k, float max_d2, int* d_idx, float* d_d2, uint32_t* d_cnt) {
+  CB_CHECK(k >= 1 && k <= kMaxK, CB_ERR_UNSUPPORTED, "k must be in [1, 256]");
+  const size_t n = c->n;
+  if (n == 0) return CB_OK;
+  const Rigid T = rigid_from_t12(nullptr);
+  const int blocks = (int)std::max<size_t>(1, std::min<size_t>((size_t)ctx->sm_count * 8, (n + kBlock - 1) / kBlock));
+  const GridView g = grid_view(c);
+  if (k <= 4)
+    knn_k_kernel<4><<<blocks, kBlock, 0, ctx->stream>>>(g, c->d_pts, (uint32_t)n, T, k, max_d2, d_idx, d_d2, d_cnt);
+  else if (k <= 16)
+    knn_k_kernel<16><<<blocks, kBlock, 0, ctx->stream>>>(g, c->d_pts, (uint32_t)n, T, k, max_d2, d_idx, d_d2, d_cnt);
+  else if (k <= 32)
+    knn_k_kernel<32><<<blocks, kBlock, 0, ctx->stream>>>(g, c->d_pts, (uint32_t)n, T, k, max_d2, d_idx, d_d2, d_cnt);
+  else if (k <= 64)
+    knn_k_kernel<64><<<blocks, kBlock, 0, ctx->stream>>>(g, c->d_pts, (uint32_t)n, T, k, max_d2, d_idx, d_d2, d_cnt);
+  else if (k <= 128)
+    knn_k_kernel<128><<<blocks, kBlock, 0, ctx->stream>>>(g, c->d_pts, (uint32_t)n, T, k, max_d2, d_idx, d_d2, d_cnt);
+  else
+    knn_k_kernel<256><<<blocks, kBlock, 0, ctx->stream>>>(g, c->d_pts, (uint32_t)n, T, k, max_d2, d_idx, d_d2, d_cnt);
+  ctx->launches += 1;
+  CB_CUDA(cudaGetLastError());
+  return CB_OK;
+}
+
+}  // namespace cb
+
 extern "C" int cb_knn_radius(cb_context* ctx, const cb_cloud* ref, const cb_cloud* qry, const float* T12, int k,
                              float max_d2, int64_t* idx, float* d2, uint32_t* counts) {
   CB_CHECK(ctx && ref && qry && idx && d2, CB_ERR_INVALID, "null argument");

@@ -124,3 +124,57 @@ def ransac_pairs(n, inlier_frac=0.3, seed=1, sigma=0.002):
 
 def frobenius(Ta, Tb):
     return float(np.linalg.norm(np.asarray(Ta, np.float64) - np.asarray(Tb, np.float64)))
+
+
+def segment_scene(n, seed=1, r_over_spacing=2.5):
+    """The segmentation benchmark scene: a ground plane, floating boxes and spheres with analytic normals, every object
+    more than r away from every other one. Returns (points, normals, radius2, objects, faces): radius2 = (2.5 x the
+    point spacing)^2; `objects` = segments of the all-true evaluator, `faces` = segments of the normals evaluator at 2
+    degrees (each box face is its own segment, a sphere stays whole: neighbouring normals differ by r / R < 2 degrees).
+    Points are shuffled."""
+    rng = np.random.default_rng(seed)
+    n_box, n_sph = 8, 4
+    # areas: ground 16 x 16 (scaled below), boxes 6 faces of edge 1.5, spheres of radius 1
+    area = 16.0 * 16.0 + n_box * 6 * 1.5**2 + n_sph * 4 * np.pi
+    h = float(np.sqrt(area / n))  # point spacing
+    parts_p, parts_n = [], []
+
+    def grid(u0, u1, v0, v1):
+        us = np.arange(u0, u1 + 1e-9, h)
+        vs = np.arange(v0, v1 + 1e-9, h)
+        U, V = np.meshgrid(us, vs, indexing="ij")
+        return U.ravel(), V.ravel()
+
+    U, V = grid(0, 16, 0, 16)
+    parts_p.append(np.stack([U, V, np.zeros_like(U)], 1))
+    parts_n.append(np.tile([0.0, 0.0, 1.0], (U.size, 1)))
+    # boxes on a 4 x 2 layout over the ground, floating 0.5 above it; spheres in a row beside them
+    for b in range(n_box):
+        o = np.array([1.0 + 3.5 * (b % 4), 1.0 + 3.5 * (b // 4), 0.5])
+        e = 1.5
+        for axis in range(3):
+            for side in (0.0, e):
+                U, V = grid(0, e, 0, e)
+                p = np.zeros((U.size, 3))
+                a1, a2 = [a for a in range(3) if a != axis]
+                p[:, axis] = side
+                p[:, a1], p[:, a2] = U, V
+                nn = np.zeros((U.size, 3))
+                nn[:, axis] = 1.0 if side > 0 else -1.0
+                parts_p.append(p + o)
+                parts_n.append(nn)
+    for s in range(n_sph):
+        c = np.array([2.0 + 3.8 * s, 11.0, 1.6])
+        m = int(4 * np.pi / h**2)
+        i = np.arange(m) + 0.5
+        phi = np.arccos(1 - 2 * i / m)
+        th = np.pi * (1 + 5**0.5) * i
+        d = np.stack([np.cos(th) * np.sin(phi), np.sin(th) * np.sin(phi), np.cos(phi)], 1)
+        parts_p.append(c + d)
+        parts_n.append(d)
+    pts = np.concatenate(parts_p).astype(np.float32)
+    nrm = np.concatenate(parts_n)
+    nrm = (nrm / np.linalg.norm(nrm, axis=1, keepdims=True)).astype(np.float32)
+    perm = rng.permutation(pts.shape[0])
+    radius2 = float(np.float32((r_over_spacing * h) ** 2))
+    return pts[perm], nrm[perm], radius2, 1 + n_box + n_sph, 1 + 6 * n_box + n_sph

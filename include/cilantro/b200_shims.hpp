@@ -390,6 +390,8 @@ public:
     return kNNInRadiusSearch(q, (size_t)nh.maxNumberOfNeighbors, nh.radius);
   }
   const ConstVectorSetMatrixMap3f& getPointsMatrixMap() const { return data_map_; }  // core/kd_tree.hpp:172-174
+  cb_cloud* b200_cloud() const { return cloud_.h; }  // the device cloud (ConnectedComponentExtraction3f)
+  size_t b200_size() const { return n_; }
 
 private:
   size_t n_;

@@ -348,6 +348,50 @@ int cb_ransac_rigid(cb_context* ctx, const cb_cloud* dst, const cb_cloud* src, u
 int cb_mean_cov(cb_context* ctx, const cb_cloud* pts, float* mean3, float* cov9);
 int cb_pca(cb_context* ctx, const cb_cloud* pts, float* mean3, float* cov9, float* evals3, float* evecs9);
 
+/* ---- connected-component segmentation -----------------------------------------------------------
+ * Replaces ConnectedComponentExtraction<float,3>::segment (clustering/connected_component_extraction.hpp:371-428) =
+ * extractConnectedComponents(tree, nh, seeds, ...) (:162-265; the overloads without seeds forward with every point as a
+ * seed) over the proximity evaluators of core/common_pair_evaluators.hpp:88-259, and getPointToClusterIndexMap
+ * (clustering/clustering_base.hpp:8-18).
+ * Neighbourhood of every point over the cloud itself, encoded as for cb_cloud_estimate_normals: k > 0, radius2 <= 0:
+ * kNN; k > 0, radius2 > 0: kNN within radius2; k == 0, radius2 > 0: every point with d2 < radius2; k == 0, radius2 <= 0:
+ * empty (every seed is a segment of its own). u -> v is an edge when v is entry j >= 1 of u's list (ascending (d2, index),
+ * the reference skips entry 0, :202) and the evaluator accepts (u, v, d2). Segments are the connected components of the
+ * undirected graph over the points reachable from the seeds along edges, seeds included.
+ * Output: segments of min_size <= size <= max_size, by size descending, equal sizes by smallest point index ascending;
+ * labels[i] = segment of point i, or *num_segments for a point in none (n entries); the points of segment s are
+ * seg_points[seg_offsets[s] .. seg_offsets[s+1]) ascending (seg_offsets has n + 1 entries, seg_points n). Point indices
+ * are positions in this cloud (index_offset is not added). The result does not depend on scheduling.
+ * seeds: NULL = every point (n_seeds ignored); repeated seeds are allowed, a seed >= n is CB_ERR_INVALID. normals: packed
+ * 3n floats in original order, NULL = the cloud's own normals (CB_ERR_INVALID for a normals evaluator when it has none);
+ * colors: packed 3n floats, required by the colour evaluators. gpu_ms (may be NULL) receives 3 floats: the device time
+ * of the call, of its neighbourhood + union stage and of its finalise stage (relabelling and the segment lists). */
+typedef enum cb_segment_evaluator {
+  CB_SEG_ALWAYS_TRUE = 0,            /* AlwaysTrueEvaluator (the default) */
+  CB_SEG_POINTS = 1,                 /* PointsProximityEvaluator: d2 < max_distance */
+  CB_SEG_NORMALS = 2,                /* NormalsProximityEvaluator: angle <= max_angle */
+  CB_SEG_COLORS = 3,                 /* ColorsProximityEvaluator: |dc|^2 < color_thresh^2 */
+  CB_SEG_POINTS_NORMALS = 4,         /* PointsNormalsProximityEvaluator (angle < max_angle) */
+  CB_SEG_POINTS_COLORS = 5,          /* PointsColorsProximityEvaluator */
+  CB_SEG_NORMALS_COLORS = 6,         /* NormalsColorsProximityEvaluator (angle < max_angle) */
+  CB_SEG_POINTS_NORMALS_COLORS = 7   /* PointsNormalsColorsProximityEvaluator (angle < max_angle) */
+} cb_segment_evaluator;
+
+typedef struct cb_segment_params {
+  int32_t k;             /* neighbourhood (see above), k <= 256 (CB_ERR_UNSUPPORTED above) */
+  float radius2;
+  int32_t evaluator;     /* cb_segment_evaluator */
+  float max_distance;    /* squared, compared with the list's d2 */
+  float max_angle;       /* radians; negative = unoriented normals: min(angle, pi - angle) <= -max_angle */
+  float color_thresh;    /* not squared (the evaluators square it) */
+  uint64_t min_size;     /* :165, default 1 */
+  uint64_t max_size;     /* :165, default SIZE_MAX */
+} cb_segment_params;
+
+int cb_cloud_segment(cb_context* ctx, cb_cloud* cloud, const cb_segment_params* prm, const uint64_t* seeds,
+                     size_t n_seeds, const float* normals, const float* colors, uint64_t* labels,
+                     uint64_t* seg_offsets, uint64_t* seg_points, size_t* num_segments, float* gpu_ms);
+
 /* transformPoints(tform, in, out) — core/space_transformations.hpp:203-216 (host in, host out). */
 int cb_transform_points(cb_context* ctx, const float* T12, const float* xyz, size_t n, float* out);
 

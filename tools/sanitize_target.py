@@ -52,6 +52,12 @@ def main():
     ds = c.grid_downsample(0.03)
     ds.estimate_normals(k=8, view_point=[0.5, 0.5, 5.0])
     ds.estimate_normals(k=0, radius2=0.06 ** 2)
+    # connected components: union passes (radius / kNN), seeded traversals, finalise
+    col = np.random.default_rng(0).uniform(0, 1, (ds.n, 3)).astype(np.float32)
+    for kw in (dict(radius2=0.06 ** 2, evaluator="normals", max_angle=0.2), dict(k=8, evaluator="points_colors",
+               max_distance=0.05 ** 2, color_thresh=0.5, colors=col)):
+        capi.segment(ctx, ds, min_size=2, **kw)
+        capi.segment(ctx, ds, seeds=np.arange(0, ds.n, 37), **kw)
     # k-means, RANSAC, PCA
     pts, cent = synth.kmeans_data(N, 16, seed=1)
     capi.kmeans_cluster(ctx, capi.Cloud(ctx, pts), cent, max_iter=3, tol=0.0)
